@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload cfg2|cfg1|cfg3|c512|c1000|cfg5|cfg5shard] [--taps default|297|2429]
+                    [--dump-outputs DIR]
 
 A "step" is ONE REFERENCE QUEUE DEPTH of the wideband stream: 64 blocks
 (queue_size, src/config.c:183) of 262144 bytes (buffer_size, src/config.c:208), each
@@ -397,6 +398,27 @@ def verify_last_block(pkg, g, wl, ids, tapsets, block_seq, get_block, ticket, sa
                     "since the group was created"}
 
 
+DUMP_BYTES = 64 << 20  # --dump-outputs budget
+
+
+def dump_outputs(pkg, g, ids, last, out_dir):
+    """--dump-outputs: what the timed path handed its callers for the last blocks of the
+    last timed step, written as out_dir/client_<c>.npy (float32 [n, 2] = re, im): client c's
+    outputs of those blocks, concatenated.  The blocks are the XLG_SLOTS whose device output
+    arenas are still live after the final wait; clients are taken in a fixed seeded order
+    while their outputs fit DUMP_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    tickets = range(last - pkg.XLG_SLOTS + 1, last + 1)
+    total = 0
+    for c in np.random.default_rng(0).permutation(len(ids)):
+        nbytes = 8 * sum(g.output_ptr(t, ids[c])[1] for t in tickets)
+        if total + nbytes > DUMP_BYTES:
+            continue
+        y = np.concatenate([g.read_output(t, ids[c]) for t in tickets])
+        np.save(os.path.join(out_dir, f"client_{c:04d}.npy"), y.view(np.float32).reshape(-1, 2))
+        total += nbytes
+
+
 # ---------------------------------------------------------------------------
 # DRAM traffic of the dominant kernel: one ncu capture taken by THIS run
 # ---------------------------------------------------------------------------
@@ -515,6 +537,8 @@ def run_stream_leg(pkg, wl, args, rank, world, local_rank, steps, warmup, partit
     host = g.profile_read(reset=True)
     barrier()
     g.wait(last)
+    if full and rank == 0 and args.dump_outputs:
+        dump_outputs(pkg, g, ids, last, args.dump_outputs)
     n_out_total = sum(g.output_ptr(last, c)[1] for c in ids)
     out = {"timed_window": (t_wall0, t_wall1), "n_out_total": n_out_total, "tapsets": tapsets,
            "partition_sms": g.partition_sms()}
@@ -692,6 +716,8 @@ def run_broadcast_leg(pkg, wl, args, rank, world, local_rank, steps, warmup):
     last = pump(g, steps * STEP_BLOCKS, False, seq)
     ms = g.timer_stop()
     barrier()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(pkg, g, ids, last, args.dump_outputs)
     ms_max = max_over_ranks(ms, world, "cuda")
     # every rank checks 4 of ITS clients of the last timed block against the oracle
     ok, worst = 1.0, 0.0
@@ -775,6 +801,8 @@ def main():
     ap.add_argument("--no-partition", action="store_true",
                     help="do not reserve 8 SMs (green context) for the oscillator pre-pass")
     ap.add_argument("--no-legs", action="store_true", help="N > 1: skip the c512 and cfg5 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last timed blocks as DIR/client_<c>.npy")
     ap.add_argument("--probe", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.probe:

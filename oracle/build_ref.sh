@@ -52,10 +52,15 @@ cp "$R/test/resources/tcp_server.config" _ref/tcp_server.config
 # --- the pinned-block queue (sdr-server_b200/host/queue_pinned.c) under the reference's own queue test ---
 $CC $STRICT $UNITY_INC -I../include -DXL_QUEUE_PAGEABLE -pthread -o _ref/test_queue_pageable $R/test/test_queue.c $UNITY_SRC $HOST/queue_pinned.c
 
+# --- the reference's src/ as it is (tests compare our headers with it and apply the patch to it) ---
+rm -rf _ref/src
+cp -r "$R/src" _ref/src
+chmod -R u+w _ref/src  # the reference may be read-only; its copies are patched
 # --- integration/cuda_cf32.patch applied to a scratch copy of the reference's src/ ---
 rm -rf _ref/patched
 mkdir -p _ref/patched
 cp -r "$R/src" _ref/patched/src
+chmod -R u+w _ref/patched/src
 patch -s -p1 -d _ref/patched < ../integration/cuda_cf32.patch
 P=_ref/patched/src
 # the patched control plane still parses (libconfig is absent: syntax only for config.c)

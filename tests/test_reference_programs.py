@@ -1,4 +1,4 @@
-"""The reference's own programs, compiled UNMODIFIED where they lie under /root/reference
+"""The reference's own programs, compiled UNMODIFIED where they lie (oracle/build_ref.sh)
 and linked against libxlating_b200.so instead of src/xlating.c + src/lpf.c (recipe:
 oracle/Makefile -> oracle/_ref/perf_xlating_b200; INTEGRATION.md section 1).
 
@@ -26,7 +26,7 @@ needs_binary = pytest.mark.skipif(not os.path.exists(PERF_B200), reason="oracle/
 def ref_program(name):
     path = os.path.join(ROOT, "oracle", "_ref", name)
     if not os.path.exists(path):
-        pytest.skip(f"oracle/_ref/{name} not built (no /root/reference when oracle/ was made)")
+        pytest.skip(f"oracle/_ref/{name} not built (the reference was absent when oracle/ was made)")
     return path
 
 
@@ -99,12 +99,11 @@ def test_pinned_queue_passes_the_reference_queue_test_on_the_gpu_box():
     assert r.returncode == 0 and unity_summary(r.stdout) == (3, 0, 0), r.stdout[-400:]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/xlating.h"), reason="needs /root/reference")
 def test_cuda_cf32_patch_applies_to_the_reference(tmp_path):
     """integration/cuda_cf32.patch is a real patch: it applies cleanly to a copy of the
     reference's src/ and touches exactly the files INTEGRATION.md names."""
     import shutil
-    shutil.copytree("/root/reference/src", tmp_path / "src")
+    shutil.copytree(ref_program("src"), tmp_path / "src")
     with open(os.path.join(ROOT, "integration", "cuda_cf32.patch")) as f:
         r = subprocess.run(["patch", "-p1", "-d", str(tmp_path)], stdin=f, capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
@@ -122,7 +121,9 @@ def test_reference_server_test_passes_on_this_library(name, optimization, tmp_pa
     `_patched_b200` with cpu_optimization = CUDA_CF32 = the patched sdr_callback submits each
     block once to the batch ABI and the dsp threads wait for tickets."""
     r = run_server_test(name, tmp_path, optimization)
-    assert r.returncode == 0 and unity_summary(r.stdout) == (11, 0, 0), r.stdout[-1200:] + r.stderr[-600:]
+    fails = "\n".join(ln for ln in r.stdout.splitlines() if ":FAIL" in ln)
+    assert r.returncode == 0 and unity_summary(r.stdout) == (11, 0, 0), (fails + "\n" + r.stdout[-1200:] +
+                                                                          r.stderr[-600:])
     if optimization:
         assert "cpu_optimization: 2" in r.stdout  # the stand-in really selected CUDA_CF32
 
@@ -179,14 +180,14 @@ def test_reference_perf_program_runs_on_the_gpu():
     print(r.stdout)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/xlating.h"), reason="needs /root/reference")
 def test_our_headers_declare_the_reference_prototypes(tmp_path):
     """One translation unit including the reference's headers AND ours: C rejects a second
     declaration of a function with a different type, so this compiles only if every
     prototype in include/xlating.h and include/lpf.h equals the reference's
     (src/xlating.h:8-38, src/lpf.h:6)."""
+    ref_src = ref_program("src")
     src = tmp_path / "both.c"
-    src.write_text('#include <stdlib.h>\n#include "/root/reference/src/lpf.h"\n#include "/root/reference/src/xlating.h"\n'
+    src.write_text(f'#include <stdlib.h>\n#include "{ref_src}/lpf.h"\n#include "{ref_src}/xlating.h"\n'
                    f'#include "{ROOT}/include/lpf.h"\n#include "{ROOT}/include/xlating.h"\n'
                    "int main(void) { return 0; }\n")
     r = subprocess.run(["gcc", "-std=c11", "-Wall", "-Werror", "-c", str(src), "-o", str(tmp_path / "both.o")],
@@ -214,26 +215,28 @@ def harness_plan(clients, fs=2016000):
     return plan
 
 
-def test_reference_dsp_workers_on_the_reference_match_the_oracle(tmp_path):
-    """Proves the harness: the files the reference's own dsp threads write (strict build)
-    are, bit for bit, what the restatement produces for the same blocks and clients."""
-    import json
+HARNESS_ON_REFERENCE = (6, 5)  # clients, blocks
 
+
+def test_reference_dsp_workers_on_the_reference_match_the_oracle():
+    """Proves the harness: the files the reference's own dsp threads write (strict build,
+    `server_harness_ref <clients> <blocks> 8 <dir> rtl dump`; their digests are stored by
+    tests/golden/record_reference_outputs.py) are, bit for bit, what the restatement
+    produces for the same blocks and clients."""
     import numpy as np
 
     from oracle import pyoracle as po
-    clients, blocks = 6, 5
-    r = run_harness("server_harness_ref", clients, blocks, 8, tmp_path, "rtl", "dump")
-    assert r.returncode == 0, r.stderr[-400:]
-    line = json.loads(r.stdout.strip().splitlines()[-1])
-    assert line["clients"] == clients and line["blocks"] == blocks and line["input_msps"] > 0
-    raw = np.fromfile(tmp_path / "input.raw", dtype=np.uint8).reshape(blocks, 262144)
+    from util import digest, harness_blocks, reference_outputs
+    want = reference_outputs()[0]["server_harness"]
+    clients, blocks = HARNESS_ON_REFERENCE
+    assert (want["clients"], want["blocks"]) == (clients, blocks)
+    raw = harness_blocks(blocks)
+    assert digest(raw) == want["input"]
     for c, (rate, offset) in enumerate(harness_plan(clients)):
         taps = po.lpf_design(1.0, 2016000, rate // 2, rate // 5)
         o = po.OracleFilter(2016000 // rate, taps, offset, 2016000, 262144)
-        want = np.concatenate([o.process_cf32("cu8", b) for b in raw])
-        got = np.fromfile(tmp_path / f"{c}.cf32", dtype=np.complex64)
-        assert got.tobytes() == want.tobytes(), c
+        got = np.concatenate([o.process_cf32("cu8", b) for b in raw])
+        assert digest(got) == want["outputs"][c], c
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="this is the no-GPU behaviour")

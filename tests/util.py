@@ -1,5 +1,11 @@
 """Shared helpers for the parity tests."""
+import hashlib
+import json
+import os
+
 import numpy as np
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 # float tolerance of the parity contract (BASELINE.json north_star: "within 1e-5
 # relative float tolerance"; SURVEY.md 0.3 shows it can only be norm-wise because
@@ -12,6 +18,36 @@ RTOL = 1e-5
 def trunc4(x):
     """(int32)(x*10000): the reference's assert_cf32 semantics (test/utils.c:179)."""
     return (np.asarray(x, dtype=np.float32) * np.float32(10000)).astype(np.int32)
+
+
+def digest(a):
+    """First 16 hex digits of the SHA-256 of an array's bytes: bit-for-bit comparison with
+    a stored output without storing the output itself."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()[:16]
+
+
+def reference_outputs():
+    """What the reference, compiled unmodified, computed for the inputs the tests generate
+    (recorded by tests/golden/record_reference_outputs.py): digests of bit-exact outputs
+    (JSON) and samples of outputs compared within a tolerance (NPZ)."""
+    with open(os.path.join(GOLDEN, "reference_outputs.json")) as f:
+        digests = json.load(f)
+    with np.load(os.path.join(GOLDEN, "reference_outputs.npz")) as z:
+        samples = {k: z[k] for k in z.files}
+    return digests, samples
+
+
+def harness_blocks(n_blocks, block_bytes=262144):
+    """The input blocks of oracle/ref_server_harness.c: one xorshift64 byte stream."""
+    m = (1 << 64) - 1
+    s = 0x9E3779B97F4A7C15
+    out = bytearray(n_blocks * block_bytes)
+    for i in range(len(out)):
+        s ^= (s << 13) & m
+        s ^= s >> 7
+        s ^= (s << 17) & m
+        out[i] = s & 0xFF
+    return np.frombuffer(bytes(out), dtype=np.uint8).reshape(n_blocks, block_bytes)
 
 
 def ramp(fmt, offset, n):
